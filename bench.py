@@ -2,10 +2,15 @@
 matching over synthetic 224x224 batches of 32 (+ the rest of the merge: LAP, partial_merge,
 PLeaS closed form over MAX_STEPS+1 batches).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one calibration batch through activation matching's accumulation loop (two model
-forwards + one fused pack/GEMM/epilogue per tap — 174 taps for ResNet-50).  ``value`` is
+forwards + one fused pack/GEMM/epilogue per tap — 174 taps for ResNet-50); ``--steps`` is the number
+of timed steps.  ``--dump-outputs DIR`` writes, after the timed steps, the cost matrices of the timed
+batches alone (warm-up excluded; summed over the ranks when N > 1), i.e. what ``activation_matching``
+with ``accumulate="sum"`` returns for those batches, as one ``DIR/cost_<group>_<axis>.npy`` per
+permutation group in float32 (both arms): the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.  ``value`` is
 calibration samples/s with the batches already resident in HBM; ``e2e`` is the same metric
 through the public ``activation_matching`` call with pinned HOST batches (H2D copy of every
 batch and the D2H read of the permutations inside the timed region).  The whole merge
@@ -67,6 +72,9 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=32, help="samples per CPU-baseline batch (32 = the config's batch)")
     ap.add_argument("--cpu-merge-steps", type=int, default=2, help="timed Adam steps of the CPU merge baseline")
     ap.add_argument("--no-extra-rooflines", action="store_true", help="skip the K4 / LAP / Cholesky / GPU-library legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the cost matrices of the timed batches alone (no warm-up) "
+                         "to DIR/<name>.npy (float32)")
     args = ap.parse_args()
     global BATCH, METRIC
     if args.batch is None:
@@ -85,6 +93,25 @@ def peaks():
         return {"hbm_gbs": p["hbm_gbs"], "bf16_tflops": p["bf16_tflops"],
                 "bf16_tflops_sustained": p.get("bf16_tflops_sustained", p["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_BUDGET = 60 * 2 ** 20  # bytes of array data written by --dump-outputs (under 64 MB with the .npy headers)
+
+
+def dump_outputs(directory, costs):
+    """Writes {(group key, axis): n x n cost matrix} as DIR/cost_<key>_<axis>.npy in float32.  Should the
+    matrices exceed DUMP_BUDGET in all, each is cut to the same fraction of its entries: a sorted sample of the
+    flattened matrix seeded by its size, so every run and every build keeps the same entries."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    arrays = {f"cost_{key}_{axis}": np.ascontiguousarray(c, dtype=np.float32) for (key, axis), c in costs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BUDGET:
+            keep = max(1, a.size * DUMP_BUDGET // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(a.size).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -163,14 +190,16 @@ def run_reference(args):
               "node": sorted((a.key, a.axis) for a in pg.node)} for k, pg in spec.items()]
     b = args.cpu_sample
     g = torch.Generator().manual_seed(123)
-    steps = min(args.steps, 20)  # ~6 s of CPU work per 32-sample step: the driver's 20 steps are honoured
+    steps = args.steps  # ~6 s of CPU work per 32-sample step
     warm = min(args.warmup, 2)
     loader = [(torch.randn(b, 3, HW, HW, generator=g), 0) for _ in range(steps + warm)]
     if warm:
         O.matching_costs(jspec, m1, m2, loader[:warm], warm, "cdist", "sum")
     t0 = time.perf_counter()
-    O.matching_costs(jspec, m1, m2, loader[warm:], steps, "cdist", "sum")
+    costs = O.matching_costs(jspec, m1, m2, loader[warm:], steps, "cdist", "sum")
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, costs)
     v = steps * b / dt
     sample = f"{steps} steps x {b} samples of {HW}x{HW} through the oracle port of activation_matching's cost loop"
     print(json.dumps({
@@ -400,6 +429,10 @@ def _run_b200(args):
         launch_mix = dict(_native.LAUNCH_COUNTS)
         for i in range(max(W, 2)):  # >= 2 so the CUDA graph of the step exists before timing
             step(i)
+        # the accumulator holds the probe and warm-up batches by now: the timed steps start from zero, so what they
+        # leave in it (and --dump-outputs writes) is the cost matrices of the K timed batches alone.  The replays
+        # read and write this buffer in place.
+        acc.flat.zero_()
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
@@ -421,6 +454,8 @@ def _run_b200(args):
             dist.barrier()
         ms = e0.elapsed_time(e1)
         clocks = sampler.stop() if sampler else None
+        if args.dump_outputs and rank == 0:  # K timed batches (x ranks); the un-captured re-runs below add to them
+            dump_outputs(args.dump_outputs, {(k.key, k.axis): c.cpu().numpy() for k, c in zip(acc.keys, acc.costs)})
         # per-launch CUDA-event timing of the statistics kernels: the timed region replays a CUDA graph
         # (events cannot bracket nodes of a replay), so the same steps are re-run un-captured with
         # events around every launch on the launching stream

@@ -11,8 +11,9 @@ needs to pin parity without the reference tree:
 
   cfg1_rn18_golden.pt   config 1: ResNet-18 pair, activation_matching on 10 batches of 32x3x224x224
                         (pleas/methods/activation_matching.py:139-177, verbatim last-batch semantics
-                        and the accumulate-fixed sum), permutations + FULL fp32 cost matrices
-                        (4.2 MB) + partial_merge ratio 0.0 state-dict digests
+                        and the accumulate-fixed sum), permutations, objectives and cost
+                        fingerprints (the 4.2 MB of matrices are not stored: the tests recompute
+                        them with the oracle port) + partial_merge ratio 0.0 state-dict digests
                         (pleas/methods/partial_matching.py:188-202)
   cfg2_rn50_golden.pt   config 2 (verbatim mode = the last batch alone): ResNet-50 pair, one batch
                         of 32x3x224x224 -> 37 permutations, objectives and cost fingerprints
@@ -112,7 +113,7 @@ def gen_cfg1(ref):
     G["am_seconds"] = time.time() - t0
     print(f"cfg1: reference activation_matching {G['am_seconds']:.1f}s")
     G["am/reference/perm"] = {axis_key(k): v.to(torch.int16) for k, v in perm.items()}
-    G["am/reference/costs"] = {axis_key(k): v.clone() for k, v in costs.items()}
+    G["am/reference/fingerprint"] = {axis_key(k): fingerprint(v) for k, v in costs.items()}
     G["am/reference/obj"] = {axis_key(k): objective(costs[k], perm[k]) for k in perm}
     t0 = time.time()
     model3 = ref.pm.partial_merge(spec, m1, m2, perm, costs, {k: 0.0 for k in spec})

@@ -414,6 +414,34 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert "workload" in d["config"]
 
 
+def test_bench_reference_arm_dumps_the_timed_batches_costs(tmp_path):
+    """`bench.py --impl reference --dump-outputs DIR` writes one float32 cost matrix per permutation group: the
+    -cdist sums over the `--steps` timed batches alone (the warm-up batch excluded), recomputed here from the
+    benchmark's seeded inputs (torch CPU generator 123, `--cpu-sample` samples of 224x224 per batch)."""
+    import numpy as np
+
+    import bench
+    from oracle import ref_oracle as O
+
+    steps, warm, b = 2, 1, 2
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--model", "resnet18",
+                          "--steps", str(steps), "--warmup", str(warm), "--cpu-sample", str(b),
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == steps
+    spec = load_spec_json("resnet18")
+    m1, m2 = bench.make_models("resnet18")
+    g = torch.Generator().manual_seed(123)
+    loader = [(torch.randn(b, 3, 224, 224, generator=g), 0) for _ in range(warm + steps)]
+    want = O.matching_costs(spec, m1, m2, loader[warm:], steps, "cdist", "sum")
+    assert sorted(f.name for f in tmp_path.iterdir()) == sorted(f"cost_{k}_{a}.npy" for k, a in want)
+    for (key, axis), c in want.items():
+        got = np.load(tmp_path / f"cost_{key}_{axis}.npy")
+        assert got.dtype == np.float32 and got.shape == c.shape, key
+        # same computation; only the host thread count may differ between the two processes
+        assert np.abs(got.astype(np.float64) - c).max() <= 1e-5 * np.abs(c).max(), key
+
+
 def test_built_library_is_sm100a_native_sass():
     """The in-tree library really is tcgen05 / TMA / redux code for sm_100a (cuobjdump -sass, no GPU
     needed): UTCHMMA + LDTM (TMEM loads) + UBLKCP (bulk copies) in the GEMM, UTCHMMA + LDGSTS in the

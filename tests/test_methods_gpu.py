@@ -657,3 +657,37 @@ def test_batchnorm_taps_derived_from_the_tap_in_front_equal_contracted_taps(mode
         # derived one is sign(s_a s_b) corr of the tap in front — the difference is the contracted path's error
         assert float((a - b).abs().max()) <= (2e-3 if mode == "corr" else 1e-5 * scale), (k, mode)
         assert_perm_or_objective(out[True][0][k].numpy(), out[False][0][k].numpy(), b.cpu().numpy(), str(k))
+
+
+def test_bench_dumps_the_timed_batches_costs(tmp_path):
+    """`bench.py --dump-outputs DIR` on the B200 arm writes the cost matrices of the `--steps` timed batches alone —
+    not the launch-count probe or the warm-up batches the benchmark's calibration runner sees first — i.e. what
+    activation_matching(accumulate="sum") returns for those batches, recomputed here from the benchmark's seeded
+    inputs (device generator 123, min(steps + warmup, 16) distinct batches, step i runs batch (warmup + i) mod that)."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import bench
+
+    steps, warm = 3, 2
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--model", "resnet18", "--steps", str(steps),
+                          "--warmup", str(warm), "--no-merge", "--no-cpu-baseline", "--no-extra-rooflines",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=root)
+    assert out.returncode == 0, out.stderr[-3000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == steps
+    P = _pkg()
+    m1, m2 = bench.make_models("resnet18", torch.device("cuda"))
+    spec = P.get_permutation_spec(m1, ((1, 3, 224, 224),))
+    gen = torch.Generator(device="cuda").manual_seed(123)
+    dev = [torch.randn(32, 3, 224, 224, generator=gen, device="cuda") for _ in range(min(steps + warm, 16))]
+    loader = [(dev[(warm + i) % len(dev)].cpu(), 0) for i in range(steps)]
+    _, costs = P.activation_matching(spec, m1, m2, loader, steps, output_costs=True, accumulate="sum")
+    assert sorted(f.name for f in tmp_path.iterdir()) == sorted(f"cost_{k.key}_{k.axis}.npy" for k in spec)
+    for k in spec:
+        got = np.load(tmp_path / f"cost_{k.key}_{k.axis}.npy")
+        want = costs[k].cpu().numpy().astype(np.float64)
+        assert got.dtype == np.float32 and got.shape == want.shape, k
+        assert np.abs(got - want).max() <= 1e-5 * np.abs(want).max(), k
