@@ -721,9 +721,11 @@ extern "C" int plb_conv2d_affine_forward(const float *const *x, const float *con
   p.trace = g_conv_trace;
   // The tensor core truncates when it adds into its fp32 accumulator (about -1e-7 relative per 16 k, gemm.cu): a
   // bias that compounds through the layers of a network (activations shrink a little in every layer).  Chains are
-  // therefore ONE box (32 k) and the promotion warps add every chain with round-to-nearest.  Measured on the
-  // ResNet-50 pair (tests/test_configs_gpu.py, worst deviation of a group's objective from the reference's):
-  // 8-box chains > 1.3e-5, 2 boxes 1.0e-5, 1 box 5.2e-6 (cuDNN fp32 forwards: ~4e-6).
+  // therefore TWO boxes (64 k), each chain's lo x hi products are issued before its hi x hi ones (they add at 2^-11
+  // of the final magnitude, so their truncation costs nothing), and the promotion warps add every chain with
+  // round-to-nearest.  Measured on the ResNet-50 pair (tests/test_configs_gpu.py, worst deviation of a group's
+  // objective from the reference's; profiles/r02_notes.md): 8-box chains in k order > 1.3e-5, 2 boxes in k order
+  // 1.0e-5, 1 box 5.2e-6, 2 boxes small products first 4.2e-6 (cuDNN fp32 forwards: ~4e-6).
   static int chain = 0;
   if (chain == 0) {
     const char *c = getenv("PLB_CONV_CHAIN");  // experiments: boxes per accumulation chain
