@@ -350,10 +350,13 @@ DIRECT_MAX_ROWS = int(os.environ.get("PLB_DIRECT_MAX_ROWS", "128"))  # 0 disable
 
 def direct_gram_eligible(x, y, axis):
     """True when a tap can use the fused narrow-tap kernel (plb_gram_direct): both operands fp32,
-    contiguous, the same [outer][C][inner] geometry, C <= 128 a multiple of 8, inner a multiple of 16."""
+    contiguous, 16-byte aligned, the same [outer][C][inner] geometry, C <= 128 a multiple of 8, inner a multiple
+    of 16."""
     if DIRECT_MAX_ROWS <= 0 or x.shape != y.shape or x.dtype != torch.float32 or y.dtype != torch.float32:
         return False
     if not (x.is_contiguous() and y.is_contiguous()):
+        return False
+    if (x.data_ptr() | y.data_ptr()) & 15:  # plb_gram_direct refuses unaligned operands; the packed path takes them
         return False
     outer, rows, inner = as_rows_view(x, axis)
     return rows <= min(DIRECT_MAX_ROWS, 128) and rows % 8 == 0 and inner % 16 == 0 and outer * inner >= 256
@@ -431,8 +434,19 @@ def choose_tma_splits(tiles, cta_group, total_boxes, tile_elems, sms):
     return best
 
 
+# Longest contraction one work item of plb_gram_tma walks, whatever split count the fill model or the caller asks
+# for.  An item accumulates in fp32 before its sums reach fp64 (the Gram in the promotion registers once per chain,
+# the row moments per converter lane, 4 values per box), and a long fp32 sum stagnates: measured on a B200 with
+# post-ReLU data, one item over K = 2^25 is off by 5e-5 in the Gram and 1.5e-3 in the sums of squares, and an item of
+# 14 364 boxes (what the fill model picks for C = 256, K = 2^25) by 2.6e-6 in the sums of squares; items of up to
+# 890 boxes stay below 7e-7 and 1e-7.  Taps of a batch of 32 walk at most ~90 boxes per item, so the cap never binds
+# there.
+TMA_MAX_K_PER_ITEM = 512 * 32
+
+
 class TmaGramPlan:
-    """TMA-fed fused cross-Gram of one tap (any width): partial tiles + the finalize geometry."""
+    """TMA-fed fused cross-Gram of one tap (any width): partial tiles + the finalize geometry.  ``splits`` (default:
+    ``choose_tma_splits``) is raised where needed so that no work item walks more than TMA_MAX_K_PER_ITEM of K."""
 
     def __init__(self, rows, outer, inner, device, pool=None, splits=None):
         self.M = self.N = rows
@@ -444,6 +458,7 @@ class TmaGramPlan:
         tile_elems = (self.ld_m // self.m_tiles) * self.bn
         self.splits = splits if splits is not None else \
             choose_tma_splits(tiles, self.cta_group, total_boxes, tile_elems, num_sms(device))
+        self.splits = max(self.splits, -(-total_boxes * 32 // TMA_MAX_K_PER_ITEM))
         need = self.splits * self.ld_m * self.ld_n
         self.partial = pool.empty(need) if pool is not None else torch.empty(need, dtype=torch.float32, device=device)
         self.alg_flops = 2.0 * rows * rows * K
