@@ -354,6 +354,33 @@ class _Tap:
 # the Gram, row sums and sums of squares of the tap in front of it (plb_cross_finalize_grouped, n_affine).  On a
 # ResNet-50 pair that is 53 of the 174 taps.  PLB_BN_AFFINE=0 contracts every tap.
 BN_AFFINE = os.environ.get("PLB_BN_AFFINE", "1") == "1"
+# A derived tap inherits the conditioning of the tap in front.  Per unit, its error is the error of that tap's Gram
+# and row moments (relative to |x|) times |s|: it grows like kappa = sqrt(1 + mean^2 / var) of the convolution output,
+# while the contracted BatchNorm output is conditioned by its own mean and spread, kappa' = sqrt(1 + beta^2 / gamma^2).
+# A BatchNorm tap is derived only while max(kappa / kappa') over model 1's units times the same over model 2's stays at
+# or below this bound; above it the tap is contracted like any other, and the convolution in front of it runs unfused.
+# Measured on a B200 (tests/test_finalize_gpu.py, RESULTS.md): at a product of 2.08 the derived statistic reaches 0.53
+# of the contracted route's error bar, at 2.6 it is 1.4 times over it, and from there it grows like 0.6-0.8 times the
+# product.  Random-init networks sit at 1; BatchNorm statistics calibrated on data reach 3 to 7 behind a ReLU.
+BN_AFFINE_MAX_GROWTH = 2.0
+
+
+def affine_growth(running_mean, running_var, eps, weight, bias):
+    """max over units of kappa / kappa' of an eval-mode BatchNorm (see BN_AFFINE_MAX_GROWTH); a unit with gamma = 0
+    outputs a constant, which the derivation reproduces exactly, and counts 0."""
+    m, v = running_mean.detach().double(), running_var.detach().double()
+    k2 = 1.0 + m * m / (v + eps)
+    g2 = weight.detach().double() ** 2 if weight is not None else torch.ones_like(m)
+    b2 = bias.detach().double() ** 2 if bias is not None else torch.zeros_like(m)
+    r2 = torch.where(g2 > 0, k2 * g2 / (g2 + b2), torch.zeros_like(k2))
+    return float(r2.max().sqrt())  # NaN statistics give NaN: never derived
+
+
+def _bn_derivable(bn_a, bn_b):
+    """True when the taps of this BatchNorm pair may be derived from the tap in front (BN_AFFINE_MAX_GROWTH)."""
+    growth = affine_growth(bn_a.running_mean, bn_a.running_var, bn_a.eps, bn_a.weight, bn_a.bias) * \
+        affine_growth(bn_b.running_mean, bn_b.running_var, bn_b.eps, bn_b.weight, bn_b.bias)
+    return growth <= BN_AFFINE_MAX_GROWTH
 
 
 def _bn_scale_shift(bn):
@@ -460,19 +487,34 @@ class CrossAccumulator:
         n = self.costs[self.group_of[node.name, axis]].shape[0]
         if mods[0].num_features != n or mods[1].num_features != n:
             return False
+        # an ill-conditioned derivation is refused: the tap is contracted, and _conv_fusion (which asks here first)
+        # leaves the convolution in front unfused, since the BatchNorm output it would skip storing is now read
+        if not _bn_derivable(*mods):
+            return False
         if not check_only:
             self.taps[self.tap_index[parent.name, axis]].affine.append(mods)
         return True
 
+    def affines_admitted(self):
+        """True while every derived tap's BatchNorm pair still passes BN_AFFINE_MAX_GROWTH.  A derived tap cannot be
+        switched to contraction in place (its BatchNorm output may not even be stored), so statistics that moved
+        past the bound after the graph was built need a new graph."""
+        return all(all(_bn_derivable(a, b) for a, b in t.affine) for t in self.taps
+                   if t.affine and tuple((_bn_key(a), _bn_key(b)) for a, b in t.affine) != t.aff_key)
+
     def refresh_affines(self):
         """(Re)computes the derived taps' scale / shift vectors when the BatchNorm tensors changed (in place:
-        captured graphs and epilogue tables keep pointing at the same buffer)."""
+        captured graphs and epilogue tables keep pointing at the same buffer).  Raises when the new statistics no
+        longer admit a derivation (affines_admitted)."""
         for t in self.taps:
             if not t.affine:
                 continue
             key = tuple((_bn_key(a), _bn_key(b)) for a, b in t.affine)
             if key == t.aff_key:
                 continue
+            if not all(_bn_derivable(a, b) for a, b in t.affine):
+                raise RuntimeError(f"tap {t.name}: the BatchNorm statistics behind it no longer admit a derived tap "
+                                   "(BN_AFFINE_MAX_GROWTH); build a new CalibrationRunner")
             parts = []
             for a, b in t.affine:
                 sa, ta = _bn_scale_shift(a)
@@ -846,7 +888,9 @@ def _get_runner(spec, model1, model2, mode, accumulate, use_cuda_graph):
     hit = _RUNNER_CACHE.get(key) if RUNNER_CACHE else None
     if hit is not None:
         runner, (refs, old_fp) = hit
-        if refs[0]() is model1 and refs[1]() is model2 and old_fp == fp:
+        # BatchNorm statistics updated in place keep the fingerprint: a derived tap they no longer admit needs a new
+        # graph, in which that tap is contracted
+        if refs[0]() is model1 and refs[1]() is model2 and old_fp == fp and runner.acc.affines_admitted():
             runner.acc.flat.zero_()
             return runner
     clear_caches()  # at most one runner is kept: its graph pools hold several GB

@@ -646,3 +646,47 @@ def test_runner_cache_fingerprints_detect_what_invalidates_a_captured_graph():
     assert AM._model_fingerprint(m) != fp
     spec = P.get_permutation_spec(m, ((1, 3, 16, 16),))
     assert AM._spec_fingerprint(spec) == AM._spec_fingerprint(P.get_permutation_spec(m, ((1, 3, 16, 16),)))
+
+
+def test_batchnorm_derivation_bound():
+    """BN_AFFINE_MAX_GROWTH admits a derived BatchNorm tap while max(kappa / kappa') of one model times the other's
+    stays within the bound: kappa^2 = 1 + mean^2 / (var + eps) of the convolution output, kappa'^2 = 1 + beta^2 /
+    gamma^2 of the BatchNorm output."""
+    import importlib
+
+    AM = importlib.import_module("pleas_merging_b200.methods.activation_matching")
+
+    def bn(mean, var, gamma, beta, affine=True):
+        m = torch.nn.BatchNorm2d(len(mean), affine=affine, eps=0.0).eval()
+        m.running_mean.copy_(torch.tensor(mean))
+        m.running_var.copy_(torch.tensor(var))
+        if affine:
+            m.weight.data.copy_(torch.tensor(gamma))
+            m.bias.data.copy_(torch.tensor(beta))
+        return m
+
+    def growth(m):
+        return AM.affine_growth(m.running_mean, m.running_var, m.eps, m.weight, m.bias)
+
+    fresh = torch.nn.BatchNorm2d(64).eval()  # random init: mean 0, var 1, gamma 1, beta 0
+    assert growth(fresh) == 1.0 and AM._bn_derivable(fresh, fresh)
+    assert AM.BN_AFFINE_MAX_GROWTH >= 1.0
+    assert growth(bn([3.0, 0.0], [1.0, 4.0], [1.0, 1.0], [0.0, 0.0])) == pytest.approx(10 ** 0.5)   # worst unit
+    assert growth(bn([3.0], [1.0], [2.0], [6.0])) == pytest.approx(1.0)                             # beta/gamma = mean/sd
+    assert growth(bn([0.0], [1.0], [-1.0], [1.0])) == pytest.approx(0.5 ** 0.5)                      # sign of gamma
+    assert growth(bn([5.0], [1.0], [0.0], [1.0])) == 0.0             # gamma = 0: a constant output, derived exactly
+    assert growth(bn([2.0], [4.0], None, None, affine=False)) == pytest.approx(2 ** 0.5)
+    assert not AM._bn_derivable(bn([float("nan")], [1.0], [1.0], [0.0]), fresh)
+    b = AM.BN_AFFINE_MAX_GROWTH
+    edge = bn([(b - 1.0) ** 0.5], [1.0], [1.0], [0.0])                # kappa = sqrt(b) on both sides
+    assert AM._bn_derivable(edge, edge)
+    worse = bn([(1.01 * b - 1.0) ** 0.5], [1.0], [1.0], [0.0])
+    assert not AM._bn_derivable(worse, worse)
+    assert AM._bn_derivable(worse, bn([0.0], [1.0], [1.0], [1.0]))   # the other model's kappa' = sqrt(2) makes room
+
+    from oracle import tinynet
+
+    m1, m2 = tinynet.make_pair(12, 10)  # perturbed statistics around mean 0, var 1: every BatchNorm stays derived
+    for (_, a), (_, c) in zip(((n, m) for n, m in m1.named_modules() if isinstance(m, torch.nn.BatchNorm2d)),
+                              ((n, m) for n, m in m2.named_modules() if isinstance(m, torch.nn.BatchNorm2d))):
+        assert AM._bn_derivable(a, c)
